@@ -1,6 +1,6 @@
 #!/usr/bin/env python
 """Reference arm of bench.py: times the UNMODIFIED reference (yeyupiaoling/VoiceprintRecognition-Pytorch, mvector 1.1.1,
-installed with `pip install --no-deps --target baseline/_ref /root/reference`) through its OWN public API --
+installed into oracle/_ref by build(), oracle/reference.py) through its OWN public API --
 ``mvector.predict.MVectorPredictor(configs, model_path, use_gpu).predict_batch(list of numpy waveforms)``
 (predict.py:231-265) -- on the box's host cores (``--device cpu``) or, for the same-box GPU-library bar, on cuda with the
 stock PyTorch eager kernels (cuDNN / cuBLAS; ``--device cuda``).  None of this repo's code is on that path.
@@ -58,7 +58,7 @@ def synth_waves(lens, seed):
 
 def main():
     spec = json.load(open(sys.argv[1]))
-    ref_root = spec.get('ref_root') or os.path.join(HERE, '_ref')
+    ref_root = spec.get('ref_root') or os.path.join(os.path.dirname(HERE), 'oracle', '_ref')
     if not os.path.isdir(os.path.join(ref_root, 'mvector')):
         print(json.dumps({'unavailable': f'no reference install at {ref_root}'}))
         return
@@ -143,7 +143,7 @@ def main():
             break
     out = {'emb_per_s': len(waves) * done / el, 'ms_per_step': 1e3 * el / done, 'steps': done, 'n_utts': len(waves),
            'elapsed_s': el, 'device': device, 'threads': threads, 'torch': torch.__version__, 'mode': mode,
-           'api': 'mvector.predict.MVectorPredictor.predict_batch (unmodified reference, baseline/_ref)'}
+           'api': 'mvector.predict.MVectorPredictor.predict_batch (unmodified reference, oracle/_ref)'}
     if device == 'cuda':
         out['tf32'] = {'cudnn': torch.backends.cudnn.allow_tf32, 'matmul': torch.backends.cuda.matmul.allow_tf32}
         out['gpu'] = torch.cuda.get_device_name(0)

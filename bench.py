@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- embeddings/sec of the waveform -> front-end -> backbone -> embedding path on the BASELINE.json configs.
 
-    python bench.py [--config c2|c3|c4|c5] [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--config c2|c3|c4|c5] [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -24,8 +24,9 @@ Timed quantities (CUDA events on the launching stream, max over ranks, barrier +
              events by vp_embed_profiled on extra steps after the timed region): algorithmic FLOPs / its launch time vs
              the measured dense bf16 tensor peak of MEASURED_PEAKS.json (burst figure: the kernel is timed alone);
              `whole_step` uses the sustained figure
-  cpu_baseline : the UNMODIFIED reference (baseline/_ref) through its own MVectorPredictor.predict_batch on the box's
-             host cores, bounded sample, separate process (falls back to the oracle port only if baseline/_ref is missing)
+  cpu_baseline : the UNMODIFIED reference (oracle/_ref, installed by build()) through its own
+             MVectorPredictor.predict_batch on the box's host cores, bounded sample, separate process (falls back to the
+             oracle port only if oracle/_ref is missing)
   gpu_eager_baseline : the same reference on the same GPU with stock PyTorch eager kernels (cuDNN / cuBLAS), TF32 as
              shipped and off, with its parity error against the reference's CPU fp32 result -- context, not the target
 `--impl reference` runs the reference arm alone and prints the same JSON line with "impl": "reference".
@@ -110,6 +111,17 @@ def save_weights(cfg, td):
     return sd
 
 
+def write_dumps(path, arrays):
+    """--dump-outputs: one float32 DIR/<name>.npy per timed path, what a caller received from its last timed step
+    (at most 2048 x 192 floats each)."""
+    if not path:
+        return
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + '.npy'), np.ascontiguousarray(a, dtype=np.float32))
+
+
 def cpu_model():
     try:
         with open('/proc/cpuinfo') as f:
@@ -122,7 +134,8 @@ def cpu_model():
 # reference arm: the unmodified reference in a separate process (baseline/ref_driver.py)
 # ------------------------------------------------------------------------------------------------------------------
 def ref_available():
-    return os.path.isdir(os.path.join(ROOT, 'baseline', '_ref', 'mvector'))
+    from oracle import reference
+    return reference.installed()
 
 
 def run_ref_driver(cfg, model_dir, lens, seed, device='cpu', steps=1, warmup=1, budget_s=0.0, tf32=None, mode='predict_batch',
@@ -151,7 +164,7 @@ def run_ref_driver(cfg, model_dir, lens, seed, device='cpu', steps=1, warmup=1, 
 
 
 def port_pass(cfg, sd, waves):
-    """Fallback when baseline/_ref is absent: the oracle port of predict.py:244-264 (kind = "port")."""
+    """Fallback when oracle/_ref is absent: the oracle port of predict.py:244-264 (kind = "port")."""
     import numpy as np
     import torch
     from oracle import frontend as ofe
@@ -177,9 +190,9 @@ def run_reference_arm(args, cfg):
         if ref_available():
             out = run_ref_driver(cfg, td, lens, 4321, device='cpu', steps=args.steps, warmup=max(args.warmup, 1))
             kind = 'reference'
-            sample += '; unmodified reference MVectorPredictor.predict_batch (baseline/_ref), default batch_size 32, autograd on as shipped'
+            sample += '; unmodified reference MVectorPredictor.predict_batch (oracle/_ref), default batch_size 32, autograd on as shipped'
         else:
-            out = {'unavailable': 'baseline/_ref missing'}
+            out = {'unavailable': 'oracle/_ref missing'}
         if 'unavailable' in out:
             import torch
             kind = 'port'
@@ -353,7 +366,9 @@ def run_gpu_arm(args, cfg):
             dist.barrier()
             torch.cuda.synchronize()
 
-    def timed(step_fn, steps, warmup, sampler=None):
+    dumps = {}
+
+    def timed(step_fn, steps, warmup, sampler=None, dump=None):
         for i in range(warmup):
             step_fn(i)
         sync_all()
@@ -362,11 +377,13 @@ def run_gpu_arm(args, cfg):
             sampler.mark_start()
         e0.record()
         for i in range(steps):
-            step_fn(warmup + i)
+            out = step_fn(warmup + i)
         e1.record()
         sync_all()
         if sampler:
             sampler.mark_end()
+        if dump and args.dump_outputs and rank == 0:     # copied now: later steps reuse the output buffers
+            dumps[dump] = out.cpu().numpy() if torch.is_tensor(out) else np.array(out)
         ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
         if world > 1:
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
@@ -374,16 +391,17 @@ def run_gpu_arm(args, cfg):
 
     mark('programs built, starting timed region')
     clocks = ClockSampler(local) if rank == 0 else None
-    ms_res = timed(step_resident, args.steps, args.warmup, clocks)
+    ms_res = timed(step_resident, args.steps, args.warmup, clocks, dump='embeddings')
     clk = clocks.stop() if clocks else None
     mark(f'resident timing done: {ms_res:.2f} ms')
     if args.light:
         if rank == 0:
+            write_dumps(args.dump_outputs, dumps)
             print(json.dumps({'light': True, 'config': args.config, 'ms_per_step': ms_res / args.steps, 'note': 'not a bench value'}))
         if world > 1:
             dist.destroy_process_group()
         return
-    ms_e2e = timed(step_e2e, args.steps, max(args.warmup, 3))
+    ms_e2e = timed(step_e2e, args.steps, max(args.warmup, 3), dump='e2e_embeddings')
     mark(f'e2e timing done: {ms_e2e:.2f} ms')
 
     # consistency of the two paths on this rank: resident and host-staged results of the same batch (same kernels, same
@@ -433,7 +451,7 @@ def run_gpu_arm(args, cfg):
             return mdist.gather_embeddings(loc_pin, n_glob, out=emb_all).cpu()
 
         try:                                             # an extra figure: a (rank-symmetric) failure must not take the line down
-            ms_pin = timed(step_pinned, args.steps, max(args.warmup, 3))
+            ms_pin = timed(step_pinned, args.steps, max(args.warmup, 3), dump='pinned_embeddings')
             e_pin = step_pinned(i_chk).to(dev)
             sync_all()
             dis_pin = float(((e_res - e_pin).norm(dim=1) / e_res.norm(dim=1)).max())
@@ -575,6 +593,7 @@ def run_gpu_arm(args, cfg):
                 'roofline': roof}
         if world == 1 and not args.no_baselines:
             line.update(side_baselines(cfg, td, sd, pred, dev))
+        write_dumps(args.dump_outputs, dumps)
         print(json.dumps(line))
     if world > 1:
         dist.barrier()
@@ -601,10 +620,10 @@ def side_baselines(cfg, td, sd, pred, dev):
             out['cpu_baseline'] = {'value': r['emb_per_s'], 'unit': 'emb/s', 'cores': r['threads'], 'kind': 'reference',
                                    'cpu_model': r.get('cpu_model'),
                                    'sample': f'{what}, {r["steps"]} passes in {r["elapsed_s"]:.1f} s; unmodified reference '
-                                             'MVectorPredictor.predict_batch (baseline/_ref) in a separate process, autograd on as shipped'}
+                                             'MVectorPredictor.predict_batch (oracle/_ref) in a separate process, autograd on as shipped'}
             ref = np.load(emb_path)
     waves = synth_waves(lens, seed)
-    if ref is None:                                     # baseline/_ref missing: oracle port, labelled as such
+    if ref is None:                                     # oracle/_ref missing: oracle port, labelled as such
         torch.set_num_threads(max((os.cpu_count() or 2) // 2, 1))
         port_pass(cfg, sd, waves)
         t0, reps = time.perf_counter(), 0
@@ -655,10 +674,18 @@ def main():
                     'baselines / per-op profile; the JSON line is NOT a bench value')
     ap.add_argument('--no-baselines', action='store_true', help='skip the cpu / gpu-eager reference side runs')
     ap.add_argument('--dump-ops', default=None, help='write the per-op device-time profile (JSON) to this path')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='b200 arm only: after the timed steps, write the embeddings each timed path returned in its last '
+                         'step as DIR/<path>.npy (float32); the inputs depend only on the arguments, so two builds '
+                         'compare output for output')
     args = ap.parse_args()
     cfg = CONFIGS[args.config]
     if args.steps is None:
         args.steps = cfg['steps'] if args.impl == 'b200' else 5
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl != 'b200':
+        ap.error('--dump-outputs applies to the b200 arm only')
     if args.impl == 'reference':
         run_reference_arm(args, cfg)
     else:

@@ -5,6 +5,8 @@ import sys
 import numpy as np
 import pytest
 
+from golden_data import arrays_sha256
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
@@ -31,7 +33,15 @@ def manifest():
 
 
 def load_golden(name):
+    """Arrays of tests/golden/<name>.npz and the weights they were made with.  A fixture whose weights would take it past
+    1 MB stores ``sd_sha256`` instead of ``sd/*``: the weights are regenerated from the manifest's seed and must match."""
     import torch
     z = np.load(os.path.join(GOLDEN, name + '.npz'))
     sd = {k[3:]: torch.from_numpy(z[k]) for k in z.files if k.startswith('sd/')}
+    if 'sd_sha256' in z.files:
+        from oracle import models as om
+        with open(os.path.join(GOLDEN, 'manifest.json')) as f:
+            m = json.load(f)[name]
+        sd = om.random_state_dict(m['model'], m['feature_dim'], seed=m['seed'], **m['model_args'])
+        assert arrays_sha256(sd.items()) == str(z['sd_sha256']), f'{name}: seeded weights differ from the golden run'
     return z, sd

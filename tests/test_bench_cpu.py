@@ -1,5 +1,5 @@
 """CPU checks of the measurement harness: the synthetic workloads of bench.py are deterministic and identical in both
-arms, the reference arm really drives the UNMODIFIED reference (baseline/_ref) in its own process, and the host-path chunk
+arms, the reference arm really drives the UNMODIFIED reference (oracle/_ref, installed by build()) in its own process, and the host-path chunk
 planner cuts batches at wave boundaries."""
 import json
 import os
@@ -30,8 +30,8 @@ def test_synthetic_workloads_are_deterministic_and_shared_by_both_arms():
     assert abs(float(np.concatenate(a).std()) - 0.1) < 0.01
 
 
-@pytest.mark.skipif(not os.path.isdir(os.path.join(ROOT, 'baseline', '_ref', 'mvector')),
-                    reason='baseline/_ref (pip install --target of the reference) not present')
+@pytest.mark.skipif(not os.path.isdir(os.path.join(ROOT, 'oracle', '_ref', 'mvector')),
+                    reason='oracle/_ref not installed: build() found no checkout of the reference')
 def test_reference_arm_runs_the_unmodified_reference():
     r = subprocess.run([sys.executable, os.path.join(ROOT, 'bench.py'), '--impl', 'reference', '--config', 'c2', '--steps', '1',
                         '--warmup', '1'], capture_output=True, text=True, timeout=600, cwd=ROOT,

@@ -222,7 +222,7 @@ def test_predict_batch_sharded_two_ranks_one_gpu(feature):
     _run_sharded(2, 'gloo', feature, same_gpu=True)
 
 
-@pytest.mark.skipif(torch.cuda.device_count() < 2, reason='needs 2 GPUs (gpurun --gpus 2)')
+@pytest.mark.skipif(torch.cuda.device_count() < 2, reason='needs 2 GPUs')
 @pytest.mark.parametrize('feature', ['Fbank', 'MFCC'])
 def test_predict_batch_sharded_nccl_two_gpus(feature):
     """One process per GPU over NCCL: the sharded result equals the single-process predict_batch bit for bit."""

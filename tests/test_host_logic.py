@@ -10,6 +10,8 @@ import numpy as np
 import pytest
 import torch
 
+from golden_data import arrays_sha256, diarization_vad
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -439,7 +441,9 @@ def test_diarization_glue_matches_reference_golden():
     from mvector.infer_utils.speaker_diarization import SpeakerDiarization, SpectralCluster
     z = np.load(os.path.join(os.path.dirname(__file__), 'golden', 'diarization.npz'))
     sd = SpeakerDiarization()
-    vad = [[float(z[f'vad{i}_t'][0]), float(z[f'vad{i}_t'][1]), z[f'vad{i}_x']] for i in range(int(z['n_vad']))]
+    vad = diarization_vad(np.random.RandomState(3))
+    assert [[s[0], s[1]] for s in vad] == [z[f'vad{i}_t'].tolist() for i in range(int(z['n_vad']))]
+    assert arrays_sha256((str(i), s[2]) for i, s in enumerate(vad)) == str(z['vad_x_sha256'])
     sd._check_audio_list(vad)
     chunks = sd._chunk(vad)
     assert np.array_equal(np.array([[c[0], c[1]] for c in chunks]), z['chunk_times'])
